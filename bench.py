@@ -27,6 +27,9 @@ KNN: 10M x 768 fp32 pre-filtered by a 2-term posting-list intersection, k=10), s
 
 --impl reference: the reference's own BruteForceIndex::topKQuery (oracle/_ref, compiled from /root/reference) on the host
 cores over the FULL 10M x 768 corpus (rank 0 only).
+
+--dump-outputs DIR (configs 2 and 3): after the timed steps, rank 0 writes what the last timed step returned — labels.npy (float64)
+and scores.npy (float32), one row per query — so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import ctypes as C
@@ -127,6 +130,27 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "reasons": sorted(reasons), "samples": len(self.samples)}
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each (queries x k) device tensor as out_dir/<name>.npy in float32 or float64 (labels below 2^53 stay exact).  Past
+    64 MB in all, a fixed seeded sample of query rows is kept, listed in rows.npy."""
+    import numpy as np
+
+    host = {name: t.cpu().numpy() for name, t in arrays.items()}
+    host = {name: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for name, a in host.items()}
+    n = next(iter(host.values())).shape[0]
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_CAP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, DUMP_CAP_BYTES // (total // n + 8)), replace=False))
+        host = {name: a[keep] for name, a in host.items()}
+        host["rows"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def knn_config(rows_total, nq, k, world, scaling, dtype="fp32", metric="cosine"):
@@ -470,6 +494,8 @@ def run_knn(args):
     st = index.stats(reset=True)
     ms_step = env.max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
     value = nq / (ms_step / 1000.0)  # true QPS: every step answers nq queries over the whole corpus
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, labels=out_labels, scores=out_scores)
 
     # ---- sustained: the same loop for >= 3 s (the short timed region above is a burst; the pass draws ~1 kW)
     sustained = None
@@ -724,6 +750,8 @@ def run_config3(args):
     st = index.stats(reset=True)
     ms_step = env.max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
     scan_us = st.scan_device_us / max(1, st.scan_launches)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, labels=out_labels, scores=out_scores)
     h_labels = np.empty((nq, k), dtype=np.uint64)
     h_scores = np.empty((nq, k), dtype=np.float64)
     for _ in range(2):
@@ -813,7 +841,12 @@ def main():
     ap.add_argument("--no-clustered", action="store_true", help="skip the clustered-corpus leg (proof tiers on non-uniform data)")
     ap.add_argument("--clustered-rows", type=int, default=2_000_000)
     ap.add_argument("--posting-docs", type=int, default=50_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's labels / scores as DIR/<name>.npy (configs 2 and 3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == 5):
+        ap.error("--dump-outputs covers the device KNN of configs 2 and 3")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -25,11 +25,10 @@ def oracle():
     return oracle_lib.port()
 
 
-@pytest.fixture(scope="session")
-def ref():
+@pytest.fixture
+def ref(request):
+    """For a test that compares with the reference: its calls into oracle/_ref answer from tests/golden/reference/."""
     import oracle_lib
 
-    r = oracle_lib.ref_vecsim()
-    if r is None:
-        pytest.skip("oracle/_ref/libvecsim_ref.so not built (needs /root/reference at build time)")
-    return r
+    with oracle_lib.reference_tape(request.module.__name__, request.node.name):
+        yield

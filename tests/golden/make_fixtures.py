@@ -3,6 +3,7 @@
 
   python tests/golden/make_fixtures.py abi       # needs /root/reference: struct layouts from its headers
   python tests/golden/make_fixtures.py postings  # transcription of the reference's own golden vectors
+  python tests/golden/make_fixtures.py reference # needs oracle/_ref: records the reference's answers (tests/golden/reference/)
 
 `postings` does not execute reference code (the posting path is Rust and no Rust toolchain exists
 here): the vectors below are copied BY VALUE from the reference's test files, each with its source
@@ -113,5 +114,17 @@ def postings():
         json.dump(POSTINGS, f, indent=1)
 
 
+# the modules whose tests take the `ref` fixture
+REFERENCE_TESTS = ["test_oracle_vecsim.py", "test_oracle_trees.py", "test_oracle_postings.py", "test_hybrid_state_machine.py"]
+
+
+def reference():
+    """Runs every test that compares with the reference on oracle/_ref itself and writes what it was asked and answered.  A GPU
+    test records its reference half before it touches the device, so on a machine without one it fails after recording."""
+    env = dict(os.environ, REFERENCE_RECORD="1")
+    tests = [os.path.join(ROOT, "tests", t) for t in REFERENCE_TESTS]
+    subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", *tests], env=env, cwd=ROOT)
+
+
 if __name__ == "__main__":
-    {"abi": abi, "postings": postings}[sys.argv[1]]()
+    {"abi": abi, "postings": postings, "reference": reference}[sys.argv[1]]()

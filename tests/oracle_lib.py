@@ -3,8 +3,16 @@
   port()        oracle/liboracle.so          our CPU restatement (plain C)
   ref_vecsim()  oracle/_ref/libvecsim_ref.so the reference's own VecSim sources, compiled in place
   ref_scorers() oracle/_ref/libscorers_ref.so the reference's src/ext/default.c
+
+oracle/_ref can only be built where the reference's sources are, so what the tests ask of it is recorded once under
+tests/golden/reference/ and replayed everywhere (reference_tape, reference_call).
 """
+import contextlib
 import ctypes as C
+import functools
+import hashlib
+import json
+import lzma
 import os
 import subprocess
 
@@ -12,6 +20,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ODIR = os.path.join(ROOT, "oracle")
+GOLDEN_REF = os.path.join(ROOT, "tests", "golden", "reference")
 
 F32, BF16, F16, I8, U8 = 0, 2, 3, 4, 5
 L2, IP, COS = 0, 1, 2
@@ -135,6 +144,147 @@ def host_has_avx512f() -> bool:
 
 
 # ---------------------------------------------------------------------------------------------
+# the reference's answers, recorded
+# ---------------------------------------------------------------------------------------------
+# A test that compares with the reference opens a tape (the `ref` fixture).  While it is open, every call marked @_recorded
+# replays the answer stored in tests/golden/reference/<module>/<test>.json.xz.  When the tape closes, a digest of the calls'
+# names and arguments (and of REF_CPU_MASK, which picks the reference's SIMD tier) checks that they were the ones the reference
+# was asked.  With REFERENCE_RECORD=1 the calls run on oracle/_ref instead and the tape is written
+# (tests/golden/make_fixtures.py reference).
+_tape = None
+
+
+def _plain(x):
+    if isinstance(x, np.generic):
+        return x.item()
+    if isinstance(x, (list, tuple)):
+        return [_plain(v) for v in x]
+    if isinstance(x, dict):
+        return {str(k): _plain(v) for k, v in sorted(x.items())}
+    return x
+
+
+def _feed(h, args):
+    def feed(x):
+        if isinstance(x, np.ndarray):
+            h.update(f"{x.dtype.str}{x.shape}".encode())
+            h.update(np.ascontiguousarray(x).tobytes())
+        elif isinstance(x, (bytes, bytearray)):
+            h.update(bytes(x))
+        elif hasattr(x, "_tape_key"):
+            feed(x._tape_key())
+        elif isinstance(x, (list, tuple)):
+            h.update(b"[")
+            for v in x:
+                feed(v)
+            h.update(b"]")
+        else:
+            h.update(json.dumps(_plain(x)).encode())
+        h.update(b"|")
+
+    feed(args)
+
+
+def _enc(x):
+    if isinstance(x, np.ndarray):
+        return {"nd": x.dtype.str, "v": x.tolist()}
+    if isinstance(x, tuple):
+        return {"tuple": [_enc(v) for v in x]}
+    if isinstance(x, list):
+        return [_enc(v) for v in x]
+    return _plain(x)
+
+
+def _dec(x):
+    if isinstance(x, dict):
+        if "tuple" in x:
+            return tuple(_dec(v) for v in x["tuple"])
+        return np.array(x["v"], dtype=x["nd"])
+    if isinstance(x, list):
+        return [_dec(v) for v in x]
+    return x
+
+
+def _live():
+    return _tape is None or _tape["record"]
+
+
+@contextlib.contextmanager
+def reference_tape(module, test):
+    """Replays (or, with REFERENCE_RECORD=1, records) the reference's answers for one test."""
+    global _tape
+    path = os.path.join(GOLDEN_REF, module, test + ".json.xz")
+    record = os.environ.get("REFERENCE_RECORD") == "1"
+    if record:
+        assert ref_vecsim() is not None and ref_scorers() is not None, "recording needs oracle/_ref (build() with the reference at hand)"
+        assert host_has_avx512f(), "the recorded answers are those of the reference's AVX-512 tier, which the tests hold the port's to"
+        rec = {"calls": [], "digest": None}
+    else:
+        if not os.path.exists(path):
+            raise FileNotFoundError(f"{path}: no recorded reference answers for this test (tests/golden/make_fixtures.py reference)")
+        with lzma.open(path, "rt") as f:
+            rec = json.load(f)
+    _tape = t = {"record": record, "calls": rec["calls"], "pos": 0, "path": path, "depth": 0, "h": hashlib.sha256()}
+    try:
+        yield
+        if not record:
+            assert t["pos"] == len(t["calls"]), f"{len(t['calls']) - t['pos']} recorded reference calls were not made: re-record {path}"
+            assert t["h"].hexdigest() == rec["digest"], f"the reference calls differ from the recorded ones: re-record {path}"
+    finally:
+        if record:  # a GPU test records its reference half before it needs the device
+            os.makedirs(os.path.dirname(path), exist_ok=True)
+            with open(path, "wb") as f:
+                f.write(lzma.compress(json.dumps({"digest": t["h"].hexdigest(), "calls": t["calls"]}, separators=(",", ":")).encode(),
+                                      preset=9 | lzma.PRESET_EXTREME))
+        _tape = None
+
+
+def reference_call(name, fn, args, kwargs=None):
+    """fn(*args, **kwargs) on the reference, or its recorded answer while a tape replays.  An argument with a _tape_key() enters the
+    digest through it."""
+    kwargs = kwargs or {}
+    t = _tape
+    if t is None or t["depth"]:
+        return fn(*args, **kwargs)
+    _feed(t["h"], [name, args, kwargs, os.environ.get("REF_CPU_MASK")])
+    if t["record"]:
+        t["depth"] += 1
+        try:
+            out = fn(*args, **kwargs)
+        finally:
+            t["depth"] -= 1
+        t["calls"].append(_enc(out))
+        return out
+    assert t["pos"] < len(t["calls"]), f"{name}: more reference calls than recorded in {t['path']}"
+    t["pos"] += 1
+    return _dec(t["calls"][t["pos"] - 1])
+
+
+def _recorded(fn):
+    """Marks a call into oracle/_ref (see reference_call)."""
+
+    @functools.wraps(fn)
+    def call(*args, **kwargs):
+        return reference_call(fn.__qualname__, fn, args, kwargs)
+
+    return call
+
+
+@_recorded
+def reference_distance(vtype, metric, dim, a, b):
+    """the reference's dispatched distance function (the tier REF_CPU_MASK leaves it)"""
+    return ref_vecsim().Ref_Distance(vtype, metric, dim, _p(np.ascontiguousarray(a)), _p(np.ascontiguousarray(b)))
+
+
+@_recorded
+def reference_normalize(blob, dim, vtype):
+    """a normalised copy of `blob` (bytes of the stored form, with the int8/uint8 norm slot) by the reference's normaliser"""
+    out = np.array(blob, copy=True)
+    ref_vecsim().Ref_Normalize(_p(out), dim, vtype)
+    return out
+
+
+# ---------------------------------------------------------------------------------------------
 # convenience wrappers
 # ---------------------------------------------------------------------------------------------
 class PortIndex:
@@ -198,29 +348,37 @@ class RefIndex:
     """The reference's BruteForceIndex through oracle/ref_shim/ref_capi.cpp."""
 
     def __init__(self, vtype, dim, metric, multi=False, block_size=1024):
-        self.L = ref_vecsim()
-        self.h = self.L.Ref_IndexNew(vtype, dim, metric, int(multi), block_size)
-        self.vtype, self.dim, self.metric = vtype, dim, metric
+        self.L = ref_vecsim() if _live() else None  # a replayed test never touches the library
+        self.h = self.L.Ref_IndexNew(vtype, dim, metric, int(multi), block_size) if self.L is not None else None
+        self.vtype, self.dim, self.metric, self.multi, self.block_size = vtype, dim, metric, multi, block_size
 
     def __del__(self):
         if getattr(self, "h", None):
             self.L.Ref_IndexFree(self.h)
             self.h = None
 
+    def _tape_key(self):  # the index's contents enter the digests through the recorded calls that made them
+        return ("RefIndex", self.vtype, self.dim, self.metric, int(self.multi), self.block_size)
+
+    @_recorded
     def add(self, blob, label):
         blob = np.ascontiguousarray(blob)
         return self.L.Ref_AddVector(self.h, _p(blob), label)
 
+    @_recorded
     def add_many(self, blobs, label0=0):
         blobs = np.ascontiguousarray(blobs)
         self.L.Ref_AddVectors(self.h, _p(blobs), blobs.shape[0], blobs.strides[0], None, label0)
 
+    @_recorded
     def delete(self, label):
         return self.L.Ref_DeleteVector(self.h, label)
 
+    @_recorded
     def size(self):
         return self.L.Ref_IndexSize(self.h)
 
+    @_recorded
     def topk(self, q, k, order=0):
         q = np.ascontiguousarray(q)
         cap = max(1, k)
@@ -230,6 +388,7 @@ class RefIndex:
         n = self.L.Ref_TopK(self.h, _p(q), k, order, cap, _p(ids), _p(scores), C.byref(code))
         return ids[:n].astype(np.int64), scores[:n]
 
+    @_recorded
     def range(self, q, radius, order=0):
         q = np.ascontiguousarray(q)
         cap = max(1, self.size())
@@ -239,13 +398,16 @@ class RefIndex:
         n = self.L.Ref_Range(self.h, _p(q), radius, order, cap, _p(ids), _p(scores), C.byref(code))
         return ids[:n].astype(np.int64), scores[:n]
 
+    @_recorded
     def distance_from(self, label, q):
         q = np.ascontiguousarray(q)
         return self.L.Ref_GetDistanceFrom(self.h, label, _p(q))
 
+    @_recorded
     def prefer_adhoc(self, subset, k, initial):
         return bool(self.L.Ref_PreferAdHoc(self.h, subset, k, int(initial)))
 
+    @_recorded
     def batches(self, q, n, order=0):
         """Drain a batch iterator n results at a time; returns a list of (ids, scores)."""
         q = np.ascontiguousarray(q)
@@ -279,9 +441,8 @@ class StreamingTopK:
         rows = np.ascontiguousarray(rows)
         nq = self.q.shape[0]
         if self.kind == "reference":
-            ref_vecsim().Ref_ScanTopKChunk(self.vtype, self.metric, self.dim, _p(rows), rows.strides[0], rows.shape[0], label0,
-                                           _p(self.q), self.q.strides[0], nq, self.k, self.threads, _p(self.ids), _p(self.scores),
-                                           _p(self.counts))
+            self.ids, self.scores, self.counts = _reference_scan_chunk(self.vtype, self.metric, self.dim, rows, label0, self.q, self.k,
+                                                                       self.threads, self.ids, self.scores, self.counts)
         else:
             port().orc_scan_topk_chunk(self.vtype, self.metric, TIER_AVX512, self.dim, _p(rows), rows.strides[0], rows.shape[0], label0,
                                        _p(self.q), self.q.strides[0], nq, self.k, self.threads, _p(self.ids), _p(self.scores),
@@ -292,6 +453,15 @@ class StreamingTopK:
         c = int(self.counts[i])
         order = np.lexsort((self.ids[i, :c], self.scores[i, :c]))
         return self.ids[i, :c][order].astype(np.int64), self.scores[i, :c][order]
+
+
+@_recorded
+def _reference_scan_chunk(vtype, metric, dim, rows, label0, q, k, threads, ids, scores, counts):
+    """Ref_ScanTopKChunk: one chunk of rows into the per-query heaps; returns the heaps' new (ids, scores, counts)."""
+    ids, scores, counts = ids.copy(), scores.copy(), counts.copy()
+    ref_vecsim().Ref_ScanTopKChunk(vtype, metric, dim, _p(rows), rows.strides[0], rows.shape[0], label0, _p(q), q.strides[0], q.shape[0], k,
+                                   threads, _p(ids), _p(scores), _p(counts))
+    return ids, scores, counts
 
 
 def synth_rows(vtype, seed, row0, nrows, dim):
@@ -580,12 +750,14 @@ def min_offset_delta(positions, virtual=None):
     return postings().orc_min_offset_delta(n, npos, flat, stride, virt)
 
 
+@_recorded
 def reference_min_offset_delta(positions, virtual=None, is_union=False):
     """the reference's own src/index_result/index_result.c:51-108 (compiled in place into libscorers_ref.so)"""
     n, npos, flat, stride, virt = _slop_args(positions, virtual)
     return ref_scorers().RefMinOffsetDelta(int(is_union), n, npos, flat, stride, virt)
 
 
+@_recorded
 def reference_hamming(payload, qdata):
     """the reference's HammingDistanceScorer (src/ext/default.c:475-497); payload None = the document has no payload"""
     return ref_scorers().RefHamming(payload, len(payload) if payload else 0, qdata, len(qdata))
@@ -621,6 +793,7 @@ def oracle_score(scorer, freqs, idf, bm25_idf, weights, agg_weight, doc_len, max
     return L.orc_score(scorer, C.byref(st), C.byref(d), slop, min_score, tanh_factor)
 
 
+@_recorded
 def reference_score(scorer, freqs, idf, bm25_idf, weights, agg_weight, doc_len, max_freq, doc_score, num_docs,
                     avg_doc_len, slop=1, min_score=0.0, tanh_factor=4, is_union=False):
     L = ref_scorers()
@@ -707,6 +880,9 @@ class ResultTree:
                                                      int(in_order)))
 
     # the reference's own code (libscorers_ref.so)
+    def _tape_key(self):
+        return (self.parent, self.kind, self.freq, self.weight, self.idf, self.bm25, self.bytes)
+
     def _ref_load(self):
         L = ref_scorers()
         rc = L.RefTreeLoad(len(self.nodes), _p(self.parent), _p(self.kind), _p(self.freq), _p(self.weight), _p(self.idf), _p(self.bm25),
@@ -714,10 +890,12 @@ class ResultTree:
         assert rc == 0
         return L
 
+    @_recorded
     def ref_score(self, scorer, doc_len, max_freq, doc_score, num_docs, avg_doc_len, slop=-1, min_score=0.0, tanh_factor=4):
         return self._ref_load().RefTreeScore(SCORER_NAMES[scorer], doc_len, max_freq, doc_score, num_docs, avg_doc_len, slop, min_score,
                                              int(tanh_factor))
 
+    @_recorded
     def ref_explain(self, scorer, doc_len, max_freq, doc_score, num_docs, avg_doc_len, slop=-1, min_score=0.0, tanh_factor=4):
         """(score, explanation) of the reference's scorer run with scrExp set; one "<depth> <string>" line per node, pre-order"""
         L = self._ref_load()
@@ -727,14 +905,17 @@ class ResultTree:
                          C.byref(sc), buf, len(buf))
         return sc.value, buf.value.decode()
 
+    @_recorded
     def ref_offsets(self, node=0):
         L = self._ref_load()
         out = np.zeros(4096, dtype=np.uint32)
         n = L.RefTreeOffsets(node, _p(out), out.size)
         return out[:n].tolist()
 
+    @_recorded
     def ref_has_offsets(self, node=0):
         return bool(self._ref_load().RefTreeHasOffsets(node))
 
+    @_recorded
     def ref_min_offset_delta(self):
         return self._ref_load().RefTreeMinOffsetDelta()

@@ -3,7 +3,7 @@
 policy review that restarts the query in ad-hoc mode (:346-370, :430-438) and ad-hoc mode (:289-335).
 
 The oracle below is the same call sequence written against the REFERENCE's own VecSim (oracle/_ref: its batch iterator,
-preferAdHocSearch, getDistanceFrom) — or the C restatement when _ref is absent — with a plain sorted docId list as the child.
+preferAdHocSearch, getDistanceFrom) with a plain sorted docId list as the child; its answers are recorded under tests/golden/reference/.
 The device side gets a B200 iterator (the result of a posting-list union) as its child.  Compared: the final mode, the
 number of batches, the docIds and the fp32 distance bits."""
 import ctypes as C
@@ -147,38 +147,43 @@ def oracle_hybrid(ref, is_ref, q_raw, q_norm, k, child_ids, forced=0, batch_size
     return mode, iters, [h[1] for h in res], np.array([h[0] for h in res], dtype=np.float32)
 
 
+def farthest_half(ref, q, n):
+    """labels 1..n as a bitmap: set for the n // 2 rows the reference ranks farthest from q"""
+    all_ids, _ = ref.topk(q, n)
+    return np.packbits(np.isin(np.arange(1, n + 1), all_ids[n // 2:]))
+
+
+@pytest.mark.usefixtures("ref")
 @pytest.mark.parametrize("scenario", ["adhoc", "batches", "batches_then_adhoc", "forced_batches_fixed_size", "few_matches"])
 def test_hybrid_state_machine_matches_the_reference_call_sequence(scenario):
     from redisearch_b200 import postings as ps
     from redisearch_b200 import vecsim as vs
 
-    is_ref = ol.ref_vecsim() is not None
-    if not is_ref:
-        pytest.skip("the batches oracle drives the reference's batch iterator (oracle/_ref)")
     n, dim, k = 60_000, 32, 10
     rows = ol.synth_rows(ol.F32, 42, 0, n, dim)
-    g = vs.VecSimIndex(vs.VecSimType_FLOAT32, dim, vs.VecSimMetric_Cosine)
     ref = ol.RefIndex(ol.F32, dim, ol.COS)
-    g.add_many(rows, label0=1)
     ref.add_many(rows, 1)
     q = ol.synth_rows(ol.F32, 43, 0, 1, dim)[0]
     qn = q.copy()
     ol.port().orc_normalize(ol._p(qn), dim, ol.F32)
     rng = np.random.default_rng(8)
-    all_ids, all_sc = ref.topk(q, n)  # every row by distance
     forced, bsz = 0, 0
     if scenario == "adhoc":
         child_ids = np.sort(rng.choice(np.arange(1, n + 1), n // 20, replace=False))  # 5 %: ad-hoc from the start
     elif scenario == "batches":
         child_ids = np.sort(rng.choice(np.arange(1, n + 1), n // 2, replace=False))  # 50 %, uncorrelated: batches finish
     elif scenario == "batches_then_adhoc":
-        child_ids = np.sort(all_ids[n // 2:])  # the FARTHEST half: batches keep finding nothing, the review switches
+        # the FARTHEST half: batches keep finding nothing, the review switches
+        child_ids = np.flatnonzero(np.unpackbits(ol.reference_call("farthest_half", farthest_half, (ref, q, n)))[:n]) + 1
     elif scenario == "forced_batches_fixed_size":
         child_ids = np.sort(rng.choice(np.arange(1, n + 1), n // 10, replace=False))
         forced, bsz = BATCHES, 500
     else:
         child_ids = np.sort(rng.choice(np.arange(1, n + 1), 4, replace=False))  # fewer matches than k
-    exp_mode, exp_iters, exp_ids, exp_sc = oracle_hybrid(ref, True, q, qn, k, child_ids, forced, bsz)
+    exp_mode, exp_iters, exp_ids, exp_sc = ol.reference_call("oracle_hybrid", oracle_hybrid, (ref, True, q, qn, k, child_ids, forced, bsz))
+
+    g = vs.VecSimIndex(vs.VecSimType_FLOAT32, dim, vs.VecSimMetric_Cosine)
+    g.add_many(rows, label0=1)
 
     pl = ps.PostingList.from_arrays(child_ids.astype(np.uint64))
     it = ps.union([pl]).into_iterator()

@@ -278,10 +278,8 @@ def test_bm25_legacy_golden_explainscore():
 
 @pytest.mark.parametrize("scorer", [ol.SCORER_BM25STD, ol.SCORER_BM25, ol.SCORER_TFIDF, ol.SCORER_TFIDF_DOCNORM,
                                     ol.SCORER_DOCSCORE, ol.SCORER_BM25STD_TANH, ol.SCORER_DISMAX])
-def test_scorers_bit_equal_to_reference_default_c(scorer):
+def test_scorers_bit_equal_to_reference_default_c(ref, scorer):
     """oracle/_ref/libscorers_ref.so is the reference's own src/ext/default.c."""
-    if ol.ref_scorers() is None:
-        pytest.skip("oracle/_ref/libscorers_ref.so not built")
     rng = np.random.default_rng(100 + scorer)
     for _ in range(300):
         n = int(rng.integers(1, 7))
@@ -304,10 +302,8 @@ def test_scorers_bit_equal_to_reference_default_c(scorer):
         assert np.float64(a).tobytes() == np.float64(b).tobytes(), (scorer, a, b)
 
 
-def test_reference_scorers_reproduce_their_own_golden():
+def test_reference_scorers_reproduce_their_own_golden(ref):
     """Sanity of the harness itself: the reference's BM25STD through libscorers_ref gives 0.54/0.52/0.51."""
-    if ol.ref_scorers() is None:
-        pytest.skip("oracle/_ref/libscorers_ref.so not built")
     g = G["bm25std_explain"]
     idf = math.log(1 + 0.5 / 3.5)
     for doc_len, total, _ in g["cases"]:
@@ -421,13 +417,11 @@ def test_numeric_codec_golden_bytes():
             assert ol.numeric_decode(ol.numeric_encode(0, v, compress))[2] == v
 
 
-def test_min_offset_delta_equals_the_reference():
+def test_min_offset_delta_equals_the_reference(ref):
     """GetSlop of the legacy scorers: the restatement against the reference's own index_result.c, and its doc-comment example."""
     assert ol.min_offset_delta([[2, 4, 8], [0, 5, 12]]) == 1           # index_result.c:47-50: abs(4-5)
     assert ol.min_offset_delta([[5]]) == 1 and ol.min_offset_delta([[], []]) == 1 and ol.min_offset_delta([[], [], []]) == 2
     assert ol.min_offset_delta([[1], [10]]) == 9 and ol.min_offset_delta([[1], [4], [8]]) == 5  # sqrt(9 + 16)
-    if ol.ref_scorers() is None:
-        pytest.skip("oracle/_ref/libscorers_ref.so not built")
     rng = np.random.default_rng(77)
     for _ in range(3000):
         n = int(rng.integers(1, 7))

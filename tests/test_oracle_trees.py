@@ -1,7 +1,8 @@
 """Result TREES (nested aggregates) in the oracle: oracle/tree_oracle.c against
   * the known answers of the reference's Merge offset iterator (RS/index_result/src/core/proximity.rs:409-470), and
   * the reference's own src/ext/default.c + src/index_result/index_result.c + src/offset_vector.c compiled in place
-    (oracle/_ref/libscorers_ref.so, RefTree*), on seeded random trees: bit-equal scores, equal offsets / GetSlop.
+    (oracle/_ref/libscorers_ref.so, RefTree*; its answers recorded under tests/golden/reference/), on seeded random trees: bit-equal
+    scores, equal offsets / GetSlop.
 CPU only."""
 import struct
 
@@ -10,9 +11,6 @@ import pytest
 
 import oracle_lib as ol
 from oracle_lib import KIND_AND, KIND_NUMERIC, KIND_OR, KIND_TERM, KIND_VIRTUAL, ResultTree
-
-needs_ref = pytest.mark.skipif(ol.ref_scorers() is None, reason="oracle/_ref/libscorers_ref.so not built (needs /root/reference)")
-
 
 def term(positions=(), freq=None, weight=1.0, idf=1.5, bm25_idf=0.7):
     return {"kind": KIND_TERM, "freq": len(positions) if freq is None else freq, "weight": weight, "idf": idf, "bm25_idf": bm25_idf,
@@ -120,7 +118,7 @@ def bits(x):
     return struct.pack("<d", x)
 
 
-@needs_ref
+@pytest.mark.usefixtures("ref")
 def test_offsets_has_offsets_and_get_slop_equal_the_reference():
     rng = np.random.default_rng(11)
     seen_nested = 0
@@ -134,7 +132,7 @@ def test_offsets_has_offsets_and_get_slop_equal_the_reference():
     assert seen_nested > 100
 
 
-@needs_ref
+@pytest.mark.usefixtures("ref")
 def test_kind_mask_quirks_equal_the_reference():
     # an aggregate of numeric children only: mask = Numeric, which is neither Virtual nor exactly Numeric|Metric -> "has offsets"
     for kids in ([{"kind": KIND_NUMERIC, "freq": 1, "weight": 1.0}], [{"kind": KIND_VIRTUAL, "freq": 1, "weight": 1.0}],
@@ -145,7 +143,7 @@ def test_kind_mask_quirks_equal_the_reference():
         assert t.min_offset_delta() == t.ref_min_offset_delta(), kids
 
 
-@needs_ref
+@pytest.mark.usefixtures("ref")
 @pytest.mark.parametrize("scorer", [ol.SCORER_BM25STD, ol.SCORER_BM25, ol.SCORER_TFIDF, ol.SCORER_TFIDF_DOCNORM, ol.SCORER_DOCSCORE,
                                     ol.SCORER_BM25STD_TANH, ol.SCORER_DISMAX])
 def test_tree_scores_are_bit_equal_to_the_reference(scorer):
@@ -177,7 +175,7 @@ def product_explain(t, scorer, doc_len, max_freq, doc_score, avg, slop, min_scor
     return sc.value, buf.value.decode()
 
 
-@needs_ref
+@pytest.mark.usefixtures("ref")
 @pytest.mark.parametrize("scorer", [ol.SCORER_BM25STD, ol.SCORER_BM25, ol.SCORER_TFIDF, ol.SCORER_TFIDF_DOCNORM, ol.SCORER_DOCSCORE,
                                     ol.SCORER_BM25STD_TANH, ol.SCORER_DISMAX])
 def test_explainscore_strings_equal_the_reference(scorer):
@@ -198,7 +196,7 @@ def test_explainscore_strings_equal_the_reference(scorer):
     assert len(shapes) >= 4 or scorer == ol.SCORER_DOCSCORE  # trees of several sizes, the early-out forms included
 
 
-@needs_ref
+@pytest.mark.usefixtures("ref")
 def test_wide_and_deep_trees_equal_the_reference():
     """up to 32 children per aggregate (the harness' and the device kernels' table size) and four levels of nesting: scores of every
     scorer bit-equal, offsets / GetSlop equal, explanations byte-equal"""

@@ -1,6 +1,6 @@
 """Pins oracle/vecsim_oracle.c (our CPU restatement) to the reference:
-  * against oracle/_ref/libvecsim_ref.so — the reference's own VecSim sources compiled in place —
-    on seeded random inputs (bit-equal where the arithmetic is order-defined), and
+  * against oracle/_ref/libvecsim_ref.so — the reference's own VecSim sources compiled in place, its answers recorded on an
+    AVX-512F host under tests/golden/reference/ — on seeded random inputs (bit-equal where the arithmetic is order-defined), and
   * against the known answers of the reference's unit tests
     (deps/VectorSimilarity/tests/unit/test_bruteforce.cpp, test_spaces.cpp).
 CPU only.
@@ -39,8 +39,6 @@ def test_fp32_distance_bit_equal_to_reference_tier(oracle, ref, metric):
     baseline, which must equal our scalar restatement (test_spaces.cpp:683-736 spirit)."""
     rng = np.random.default_rng(1234 + metric)
     for tier, mask in ((TIER_AVX512, None), (TIER_SCALAR, "avx512f,avx,avx2,sse,sse3,sse4_1,fma3,f16c")):
-        if tier == TIER_AVX512 and not ol.host_has_avx512f():
-            continue
         if mask:
             os.environ["REF_CPU_MASK"] = mask
         try:
@@ -48,7 +46,7 @@ def test_fp32_distance_bit_equal_to_reference_tier(oracle, ref, metric):
                 for _ in range(8):
                     a = rng.uniform(-1, 1, dim).astype(np.float32)
                     b = rng.uniform(-1, 1, dim).astype(np.float32)
-                    r = ref.Ref_Distance(F32, metric, dim, ol._p(a), ol._p(b))
+                    r = ol.reference_distance(F32, metric, dim, a, b)
                     o = oracle.orc_distance(F32, metric, dim, ol._p(a), ol._p(b), tier)
                     assert _bits(r) == _bits(o), (tier, dim, r, o)
         finally:
@@ -65,7 +63,7 @@ def test_int_distance_exact(oracle, ref, vtype, metric):
         for _ in range(4):
             a = _rand(rng, vtype, dim, metric)
             b = _rand(rng, vtype, dim, metric)
-            r = ref.Ref_Distance(vtype, metric, dim, ol._p(a), ol._p(b))
+            r = ol.reference_distance(vtype, metric, dim, a, b)
             o = oracle.orc_distance(vtype, metric, dim, ol._p(a), ol._p(b), TIER_SCALAR)
             assert _bits(r) == _bits(o), (dim, r, o)
 
@@ -81,7 +79,7 @@ def test_half_distance_close_to_fp32_accumulate_tier(oracle, ref, vtype, metric)
         for dim in DIMS:
             a = _rand(rng, vtype, dim, metric)
             b = _rand(rng, vtype, dim, metric)
-            r = ref.Ref_Distance(vtype, metric, dim, ol._p(a), ol._p(b))
+            r = ol.reference_distance(vtype, metric, dim, a, b)
             o = oracle.orc_distance(vtype, metric, dim, ol._p(a), ol._p(b), TIER_SCALAR)
             scale = 1.0 if metric == IP else 0.0
             assert abs(r - o) <= 1e-4 * max(abs(r), scale) + 1e-6, (dim, r, o)
@@ -99,7 +97,7 @@ def test_normalize_bit_equal(oracle, ref, vtype):
         a = np.zeros(blob.nbytes + extra, dtype=np.uint8)
         a[: blob.nbytes] = blob.view(np.uint8)
         b = a.copy()
-        ref.Ref_Normalize(ol._p(a), dim, vtype)
+        a = ol.reference_normalize(a, dim, vtype)
         oracle.orc_normalize(ol._p(b), dim, vtype)
         assert a.tobytes() == b.tobytes(), dim
 
@@ -118,11 +116,10 @@ def test_topk_matches_reference_index(oracle, ref, vtype, metric):
     os.environ["REF_CPU_MASK"] = "avx512_fp16"
     try:
         r = ol.RefIndex(vtype, dim, metric)
-        tier = TIER_AVX512 if ol.host_has_avx512f() else TIER_SCALAR
-        p = ol.PortIndex(vtype, dim, metric, tier=tier)
+        p = ol.PortIndex(vtype, dim, metric, tier=TIER_AVX512)
         _fill(r, blobs, 1)
         _fill(p, blobs, 1)
-        exact = vtype in (I8, U8) or (vtype == F32 and ol.host_has_avx512f())
+        exact = vtype in (I8, U8, F32)
         for qi in range(5):
             q = ol.to_type(rng.uniform(-1, 1, dim).astype(np.float32), vtype)
             for order in (0, 1):
@@ -143,7 +140,7 @@ def test_swap_delete_and_update_match_reference(oracle, ref):
     n, dim = 500, 16
     x = rng.uniform(-1, 1, (n, dim)).astype(np.float32)
     r = ol.RefIndex(F32, dim, L2)
-    p = ol.PortIndex(F32, dim, L2, tier=TIER_AVX512 if ol.host_has_avx512f() else TIER_SCALAR)
+    p = ol.PortIndex(F32, dim, L2, tier=TIER_AVX512)
     _fill(r, x, 0)
     _fill(p, x, 0)
     for lab in rng.choice(n, 120, replace=False).tolist():
@@ -168,7 +165,7 @@ def test_range_and_batches_match_reference(oracle, ref):
     n, dim = 2000, 32
     x = rng.uniform(-1, 1, (n, dim)).astype(np.float32)
     r = ol.RefIndex(F32, dim, L2)
-    p = ol.PortIndex(F32, dim, L2, tier=TIER_AVX512 if ol.host_has_avx512f() else TIER_SCALAR)
+    p = ol.PortIndex(F32, dim, L2, tier=TIER_AVX512)
     _fill(r, x, 1)
     _fill(p, x, 1)
     q = rng.uniform(-1, 1, dim).astype(np.float32)
@@ -238,7 +235,7 @@ def test_known_answers_spaces(oracle):
     assert oracle.orc_distance(I8, IP, dim, ol._p(ai), ol._p(ai), 0) == 1.0 - 55.0
 
 
-def test_streaming_topk_equals_the_reference_index():
+def test_streaming_topk_equals_the_reference_index(ref):
     """bench.py's parity check at the full 10M x 768 size feeds the device's own rows back chunk by chunk to
     ol.StreamingTopK (the reference's distance kernels + heap over a flat array): it must answer exactly like the
     reference's BruteForceIndex::topKQuery over the same rows, ties at the boundary included."""
@@ -253,8 +250,7 @@ def test_streaming_topk_equals_the_reference_index():
         ol.port().orc_normalize(ol._p(r), dim, ol.F32)
     ix = ol.PortIndex(ol.F32, dim, ol.IP, tier=ol.TIER_AVX512)
     ix.add_many(rows, 1)
-    kinds = ["port"] + (["reference"] if ol.ref_vecsim() is not None else [])
-    for kind in kinds:
+    for kind in ("port", "reference"):
         st = ol.StreamingTopK(ol.F32, ol.COS, dim, qs, k, 3)
         st.kind = kind
         for c in range(0, n, 7000):
