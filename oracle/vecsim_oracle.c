@@ -563,13 +563,14 @@ size_t orc_index_range(const OrcIndex *ix, const void *query, double radius, int
 double orc_index_distance_from(const OrcIndex *ix, size_t label, const void *stored_form_query) {
     LabelSlot *s = tab_find(ix, label, 0);
     if (!s) return NAN; /* brute_force_single.h:204-207 */
-    double best = INFINITY;
+    /* brute_force_multi.h:234-238: `dist = (dist < d) ? dist : d` from +inf in the label's row order, so a NaN row replaces
+     * the running value and the next row replaces the NaN: NaN exactly when the last row is NaN */
+    float best = INFINITY;
     for (uint32_t j = 0; j < s->n; j++) {
-        double d = (double)dist_row(ix, s->ids[j], stored_form_query);
-        if (s->n == 1) return d;
-        if (d < best) best = d;
+        const float d = dist_row(ix, s->ids[j], stored_form_query);
+        best = (best < d) ? best : d;
     }
-    return best;
+    return (double)best;
 }
 
 int orc_index_prefer_adhoc(const OrcIndex *ix, size_t subset, size_t k, int initial) {

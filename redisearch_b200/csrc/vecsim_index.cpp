@@ -1236,11 +1236,11 @@ double FlatIndex::distance_from(size_t label, const void *blob) {
     ok = ok && cudaMemcpyAsync(c->h_dist, c->d_dist, ids.size() * 4, cudaMemcpyDeviceToHost, c->stream) == cudaSuccess;
     ok = ok && cudaStreamSynchronize(c->stream) == cudaSuccess;
     double best = nan;
-    if (ok) { // brute_force_multi.h:224-241: min over the label's vectors
-        for (size_t i = 0; i < ids.size(); i++) {
-            const double d = (double)c->h_dist[i];
-            if (i == 0 || d < best || std::isnan(best)) best = d;
-        }
+    if (ok) { // brute_force_multi.h:234-238: the min over the label's rows, folded in their order as `(dist < d) ? dist : d`,
+              // so a NaN row is replaced by the next row and the answer is NaN only when the last row is NaN
+        float dist = std::numeric_limits<float>::infinity();
+        for (size_t i = 0; i < ids.size(); i++) dist = (dist < c->h_dist[i]) ? dist : c->h_dist[i];
+        best = (double)dist;
     }
     launches_total_ += lc.launches;
     checkin(std::move(c));
@@ -1409,11 +1409,13 @@ void FlatIndex::adhoc_distances(AdhocCtx *a, const size_t *labels, double *out, 
     ok = ok && cudaStreamSynchronize(c.stream) == cudaSuccess;
     launches_total_ += lc.launches;
     if (!ok) return;
+    // the same fold as distance_from over each label's rows in their order (brute_force_multi.h:234-238)
+    std::vector<float> dist(n, std::numeric_limits<float>::infinity());
     for (size_t i = 0; i < ids.size(); i++) {
-        const double d = (double)c.h_dist[i];
-        double &o = out[owner[i]];
-        if (std::isnan(o) || d < o) o = d;
+        float &d = dist[owner[i]];
+        d = (d < c.h_dist[i]) ? d : c.h_dist[i];
     }
+    for (size_t i = 0; i < ids.size(); i++) out[owner[i]] = (double)dist[owner[i]];
 }
 
 

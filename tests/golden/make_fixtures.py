@@ -115,7 +115,8 @@ def postings():
 
 
 # the modules whose tests take the `ref` fixture
-REFERENCE_TESTS = ["test_oracle_vecsim.py", "test_oracle_trees.py", "test_oracle_postings.py", "test_hybrid_state_machine.py"]
+REFERENCE_TESTS = ["test_oracle_vecsim.py", "test_oracle_vecsim_scan_paths.py", "test_oracle_trees.py", "test_oracle_postings.py",
+                   "test_hybrid_state_machine.py", "test_vecsim_scan_paths.py"]
 
 
 def reference():

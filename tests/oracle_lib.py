@@ -423,6 +423,34 @@ class RefIndex:
         self.L.Ref_BatchFree(it)
         return out
 
+    @_recorded
+    def batch_script(self, q, steps):
+        """One batch iterator driven by `steps`: ("next", n, order) | ("reset",) | ("has_next",) | ("add", blob, label) |
+        ("delete", label), the last two on the index while the iterator lives.  Returns one entry per step: (ids, scores) for
+        "next", a bool for "has_next", the return code for "add" / "delete", None for "reset"."""
+        q = np.ascontiguousarray(q)
+        it = self.L.Ref_BatchNew(self.h, _p(q))
+        out = []
+        for st in steps:
+            if st[0] == "next":
+                n = st[1]
+                ids = np.empty(max(1, n), dtype=np.uint64)
+                scores = np.empty(max(1, n), dtype=np.float64)
+                m = self.L.Ref_BatchNext(it, n, st[2], n, _p(ids), _p(scores))
+                out.append((ids[:m].astype(np.int64), scores[:m]))
+            elif st[0] == "reset":
+                self.L.Ref_BatchReset(it)
+                out.append(None)
+            elif st[0] == "has_next":
+                out.append(bool(self.L.Ref_BatchHasNext(it)))
+            elif st[0] == "add":
+                blob = np.ascontiguousarray(st[1])
+                out.append(self.L.Ref_AddVector(self.h, _p(blob), st[2]))
+            else:
+                out.append(self.L.Ref_DeleteVector(self.h, st[1]))
+        self.L.Ref_BatchFree(it)
+        return out
+
 
 class StreamingTopK:
     """k nearest rows of a corpus that is handed over chunk by chunk (stored-form rows, e.g. copied back from the device):
